@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- M query-points/sec of the occupancy query on a dense grid (BASELINE.json's metric).
 
-Contract (driver): `python bench.py --gpus N --steps K --warmup W` prints ONE JSON line on rank 0.
+Usage: `python bench.py --gpus N --steps K --warmup W [--dump-outputs DIR]` prints ONE JSON line on rank 0.
 Default workload = BASELINE.json configs[1] (the config the metric is quoted on): icon-filter, dense 256^3
 cell-centre lattice, one image per GPU (weak scaling).  A step = one pass of the hot path
 (HGPIFuNet.query: SMPL SDF block + feature gather + occupancy MLP + in_cube mask, through query_func) over
@@ -17,6 +17,9 @@ points and D2H of the occupancies inside the timed region), `roofline` of the do
 the other kernels of the path), `recon` (one full image per rank: filter -> Seg3dLossless engine -> marching cubes
 -> NCCL gather of the meshes to rank 0, the only collective of the path), `reference_gpu` (the reference's own
 stock-PyTorch/cuDNN encoders timed on the same GPU) and `cpu_baseline`.
+
+`--dump-outputs DIR` writes the occupancies the last timed step computed (see dump_outputs), so that two builds can
+be compared output for output: the inputs are seeded and identical from run to run.
 
 `--impl reference` times the reference's CPU path for the same metric: the oracle's port of query_func (oracle/,
 brute-force SDF in C with OpenMP + torch CPU MLP) on the host cores, on a bounded sample of the same lattice.
@@ -52,6 +55,8 @@ WORKLOADS = {
 }
 DEFAULT_WORKLOAD = "icon-filter-256"
 CPU_SAMPLE = 131072
+DUMP_BYTES = 60 << 20                # --dump-outputs writes at most this much, over all ranks
+DUMP_SEED = 1234
 
 
 def _peaks():
@@ -497,6 +502,27 @@ def reference_gpu_encoders(dev, netG, reps=3):
     return out
 
 
+def dump_outputs(out_dir, preds, image_ids, budget=DUMP_BYTES):
+    """preds[k] ([1, 1, N] on the device) of image image_ids[k] -> out_dir/preds_image<id>.npy.  When every point of
+    every image does not fit in `budget` bytes, each image keeps the same seeded random sample of its N points, so
+    that two runs with the same arguments write comparable arrays."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    if not preds:
+        return
+    n = preds[0].numel()
+    k = min(n, budget // 4 // len(preds))
+    idx = None
+    if k < n:
+        g = torch.Generator().manual_seed(DUMP_SEED)
+        idx = torch.randint(0, n, (k,), generator=g).sort().values.to(preds[0].device)
+    for i, p in zip(image_ids, preds):
+        v = p.reshape(-1)
+        v = v if idx is None else v[idx]
+        np.save(os.path.join(out_dir, f"preds_image{i:03d}.npy"), v.float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -508,7 +534,14 @@ def main():
     ap.add_argument("--grid", type=int, default=None, help=argparse.SUPPRESS)
     ap.add_argument("--no-cpu-baseline", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--no-extras", action="store_true", help="metric + e2e only (skip recon / rooflines / baselines)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the occupancies the last timed step computed to DIR/preds_image<i>.npy (float32; a "
+                         "fixed seeded sample of each image's points when all of them would exceed 60 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     wl = dict(WORKLOADS[args.workload])
     if args.grid:
         wl["grid"] = args.grid
@@ -557,10 +590,12 @@ def main():
         im.bind(netG)
         return net.query_func(cfg, netG, [im.feat], pts)
 
-    def step_resident():
+    def step_resident(keep=None):
         out = None
         for im in images:
             out = query(im, pts_dev)
+            if keep is not None:
+                keep.append(out)
         return out
 
     sampler = ClockSampler(local)
@@ -576,14 +611,18 @@ def main():
     l0 = _C.launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
+    last_step = []                            # the preds of every image in the last timed step, for --dump-outputs
     e0.record()
-    for _ in range(args.steps):
-        out = step_resident()
+    for s in range(args.steps):
+        out = step_resident(last_step if args.dump_outputs and s == args.steps - 1 else None)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = _C.launch_count() - l0
     checksum = float(out.double().sum().item()) if out is not None else 0.0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step, mine, DUMP_BYTES // world)
+    del last_step
 
     # ---- timed region 2: end to end through query_func with HOST buffers.  Every image of every step copies its
     #      points from pinned host memory and its result back; the three stages (H2D, query, D2H) of consecutive

@@ -1,146 +1,94 @@
-"""The drop-in boundary, proven on the reference's own caller: with icon_b200.overlay installed, the UNMODIFIED
-/root/reference/apps/ICON.py imports, `ICON(cfg)` builds, its netG / reconEngine / query_func are the icon_b200
-objects, every other `lib.*` name it uses is still the reference's, and `load_checkpoint`
-(lib/dataset/mesh_util.py:187-237) round-trips a synthetic checkpoint.
+"""The drop-in boundary: with icon_b200.overlay installed on an ICON checkout, the HGPIFuNet / Seg3dLossless /
+query_func / get_visibility / clean_mesh names apps/ICON.py imports are the icon_b200 objects, and every other
+`lib.*` name it uses is still the checkout's.
 
-Third-party packages the reference imports but this container lacks (pytorch_lightning, kaolin, pytorch3d, trimesh,
-...) are replaced by permissive stubs -- the SURVEY 8c recipe, generalised; they are NOT on the accelerated path.
-Runs on the CPU; skipped where /root/reference is absent (the GPU box)."""
-import importlib.abc
-import importlib.machinery
+The checkout is a stand-in built from tests/golden/overlay_layout.json (recorded from YuliangXiu/ICON by
+tests/golden/make_overlay_layout.py): the same modules, the same top-level names in the same order, the same
+`from ... import` statements between them, with a placeholder behind every name.  A module the overlay replaces
+raises when executed, so importing it proves it never runs.  Runs on the CPU."""
+import json
 import os
 import subprocess
 import sys
 import textwrap
 
-import pytest
-
-REF = "/root/reference"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "apps")), reason="reference checkout absent")
-
 SCRIPT = r'''
-import importlib.abc, importlib.machinery, importlib.util, os, sys, types
-import torch, torch.nn as nn
-REF, ROOT = sys.argv[1], sys.argv[2]
-THIS = os.path.abspath(__file__)
+import os, sys
+CHECKOUT, ROOT = sys.argv[1], sys.argv[2]
 sys.path.insert(0, ROOT)
 
-# ---- permissive stubs for absent third-party packages (never for lib.* / apps.* / icon_b200.*)
-NEVER_STUB = {"lib", "apps", "icon_b200", "oracle", "torch", "numpy", "torchvision"}
-ALWAYS_STUB = {"smplx", "turtle"}        # `smplx`: the reference vendors lib/smplx; `turtle` (a stray import) needs Tk
-STUBBED = set()
-
-class _Anything:
-    def __init__(self, *a, **k): pass
-    def __call__(self, *a, **k): return _Anything()
-    def __getattr__(self, k):
-        if k.startswith("__"): raise AttributeError(k)
-        return _Anything()
-
-class _StubModule(types.ModuleType):
-    def __getattr__(self, k):
-        if k.startswith("__"): raise AttributeError(k)
-        if self.__name__ == "pytorch_lightning" and k == "LightningModule": return nn.Module
-        return type(k, (_Anything,), {})
-
-class _StubFinder(importlib.abc.MetaPathFinder, importlib.abc.Loader):
-    """LAST on sys.meta_path: reached only for modules nothing else can import."""
-    def find_spec(self, name, path, target=None):
-        top = name.split(".")[0]
-        if top in NEVER_STUB or top.startswith("_"):
-            return None
-        if top not in STUBBED:                 # only imports made BY reference code (optional imports that installed
-            f = sys._getframe(1)               # packages guard with try/except must keep failing normally)
-            while f is not None and ("importlib" in f.f_code.co_filename or f.f_code.co_filename == THIS):
-                f = f.f_back
-            if f is None or not f.f_code.co_filename.startswith(REF):
-                return None
-        STUBBED.add(top)
-        return importlib.machinery.ModuleSpec(name, self, is_package=True)
-    def create_module(self, spec):
-        m = _StubModule(spec.name); m.__path__ = []; return m
-    def exec_module(self, module): pass
-for _n in ALWAYS_STUB:
-    sys.modules[_n] = _StubModule(_n); sys.modules[_n].__path__ = []
-sys.meta_path.append(_StubFinder())
-
 import icon_b200.overlay as OV
-OV.install(REF)
+OV.install(CHECKOUT)
 
-import apps.ICON as A                                   # the reference's file, unmodified
+import apps.ICON as A
 import lib.common.train_util as TU, lib.dataset.mesh_util as MU, lib.net as LN
-import icon_b200.net, icon_b200.engine, icon_b200.encoders, icon_b200.visibility
-assert A.__file__.startswith(REF) and TU.__file__.startswith(REF) and MU.__file__.startswith(REF)
+import icon_b200.net, icon_b200.engine, icon_b200.encoders, icon_b200.visibility, icon_b200.mesh
+assert A.__file__.startswith(CHECKOUT) and TU.__file__.startswith(CHECKOUT) and MU.__file__.startswith(CHECKOUT)
+for name in ("lib.net.HGPIFuNet", "lib.common.seg3d_lossless"):
+    assert sys.modules[name].__icon_b200_overlay__ == "replace", name
 assert A.HGPIFuNet is icon_b200.net.HGPIFuNet and LN.HGPIFuNet is icon_b200.net.HGPIFuNet
 assert LN.NormalNet is icon_b200.encoders.NormalNet and LN.VolumeEncoder is icon_b200.encoders.VolumeEncoder
 assert A.Seg3dLossless is icon_b200.engine.Seg3dLossless
 assert A.query_func is icon_b200.net.query_func and TU.query_func is icon_b200.net.query_func
 assert A.get_visibility is icon_b200.visibility.get_visibility
-import icon_b200.mesh
 assert A.clean_mesh is icon_b200.mesh.clean_mesh and MU.clean_mesh is icon_b200.mesh.clean_mesh
-# names of the patched modules that are NOT on the accelerated path are still the reference's own objects
+# names of the patched modules that are NOT on the accelerated path are still the checkout's own objects
 for name in ("SMPLX", "update_mesh_shape_prior_losses", "load_checkpoint", "cal_sdf_batch", "feat_select", "remesh"):
     assert getattr(MU, name).__module__ == "lib.dataset.mesh_util", name
 for name in ("batch_mean", "accumulate", "calc_error", "tf_log_convert", "bar_log_convert", "export_cfg"):
     assert getattr(TU, name).__module__ == "lib.common.train_util", name
     assert getattr(A, name) is getattr(TU, name), name             # `from lib.common.train_util import *` still complete
-assert TU.get_visibility is icon_b200.visibility.get_visibility    # the duplicate at train_util.py:361 as well
+assert TU.get_visibility is icon_b200.visibility.get_visibility    # train_util's own get_visibility as well
 import lib.net.FBNet as FB, lib.net.net_util as NU
 assert FB.LocalEnhancer.__module__ == "lib.net.FBNet" and NU.VGGLoss.__module__ == "lib.net.net_util"
 assert isinstance(FB.define_G(6, 3, 64, "global", 4, 9, 1, 3, "instance"), icon_b200.encoders.GlobalGenerator)
-
-# the licensed SMPL-X asset files (data/smpl_related/..., docs/installation.md:140-211) are absent offline: the
-# reference's SMPLX() constructor only np.load()s them, so it is neutralised for this test
-MU.SMPLX.__init__ = lambda self: setattr(self, "model_dir", "/nonexistent")
-from icon_b200 import config
-cfg = config.preset("icon-filter")
-cfg.merge({"lr_G": 1e-3, "sdf": False, "gpus": [0], "test_gpus": [0], "mcube_res": 256, "clean_mesh": True,
-           "batch_size": 1, "resume_path": "/tmp/_icon_b200_main.ckpt", "normal_path": "/tmp/_icon_b200_normal.ckpt"})
-model = A.ICON(cfg)
-assert type(model.netG) is icon_b200.net.HGPIFuNet and type(model.reconEngine) is icon_b200.engine.Seg3dLossless
-assert model.resolutions == [33, 65, 129, 257] and model.reconEngine._res == [33, 65, 129, 257]
-assert model.reconEngine.query_func is icon_b200.net.query_func
-
-# ---- load_checkpoint round trip (lib/dataset/mesh_util.py:187-237) with synthetic checkpoints
-from icon_b200 import synthetic as S
-sd = model.state_dict()
-main = {k: v for k, v in S.seeded_like({k: v for k, v in sd.items() if k.startswith("netG.") and "normal_filter" not in k}, 1).items()}
-for k in list(main):                       # ConvBlock registers bn4 twice (bn4 and downsample.0, net_util.py:244-251):
-    if ".downsample.0." in k:              # one parameter, two keys -- give both the same value, as a real ckpt has
-        main[k] = main[k.replace(".downsample.0.", ".bn4.")]
-main["reconEngine.b_min"] = torch.zeros(1, 1, 3)                       # must be ignored by the loader's filter
-normal = {k.replace("netG.normal_filter.", "netG."): v for k, v in
-          S.seeded_like({k: v for k, v in sd.items() if k.startswith("netG.normal_filter.")}, 2).items()}
-torch.save({"state_dict": main}, cfg.resume_path)
-torch.save({"state_dict": normal}, cfg.normal_path)
-class _CpuTorch:                       # no GPU in this container: `torch.device("cuda:0")` -> cpu, for the loader only
-    def __getattr__(self, k):
-        return (lambda *a, **kw: torch.device("cpu")) if k == "device" else getattr(torch, k)
-try:
-    MU.torch = _CpuTorch()
-    model = MU.load_checkpoint(model, cfg)
-finally:
-    MU.torch = torch
-    os.remove(cfg.resume_path); os.remove(cfg.normal_path)
-after = model.state_dict()
-for k, v in main.items():
-    if k.startswith("netG."):
-        assert torch.equal(after[k], v), k
-for k, v in normal.items():
-    assert torch.equal(after[k.replace("netG.", "netG.normal_filter.", 1)], v), k
-assert not model.netG.training
-n_main = sum(1 for k in main if k.startswith("netG."))
-print(f"OVERLAY_OK main={n_main} normal={len(normal)} keys; stubbed third-party: {sorted(STUBBED)}")
+assert FB.define_G(6, 3, 64, "local", 4, 9, 1, 3, "instance") == ("lib.net.FBNet", "define_G")
+print("OVERLAY_OK")
 '''
 
 
-def test_reference_apps_icon_imports_and_builds_under_the_overlay(tmp_path):
+def write_checkout(root, layout, replaced):
+    """One .py file per recorded module; `def` / `class` / value names become placeholders whose value (or
+    __module__) names the module that defined them."""
+    for name, mod in layout["modules"].items():
+        parts = name.split(".")
+        path = os.path.join(root, *parts) + ("/__init__.py" if mod["package"] else ".py")
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        for i in range(1, len(parts)):                 # parent packages that were not recorded
+            init = os.path.join(root, *parts[:i], "__init__.py")
+            if not os.path.exists(init):
+                open(init, "w").close()
+        if name in replaced:
+            lines = [f"raise ImportError('{name} is replaced by icon_b200.overlay and must not run')"]
+        else:
+            lines = []
+            for entry in mod["body"]:
+                kind, n = entry[0], entry[1]
+                if kind == "import":
+                    lines.append(f"from {n} import {', '.join(entry[2])}")
+                elif kind == "def":
+                    lines.append(f"def {n}(*args, **kwargs):\n    return ({name!r}, {n!r})")
+                elif kind == "class":
+                    lines.append(f"class {n}:\n    pass")
+                else:
+                    lines.append(f"{n} = ({name!r}, {n!r})")
+        with open(path, "w") as f:
+            f.write("\n".join(lines) + "\n")
+
+
+def test_overlay_on_recorded_icon_layout(tmp_path, golden_dir):
+    from icon_b200 import overlay
+    layout = json.load(open(os.path.join(golden_dir, "overlay_layout.json")))
+    replaced, patched = set(overlay._replacements()), set(overlay._patches())
+    assert (replaced | patched) <= set(layout["modules"])
+    checkout = tmp_path / "ICON"
+    write_checkout(str(checkout), layout, replaced)
     script = tmp_path / "overlay_check.py"
     script.write_text(textwrap.dedent(SCRIPT))
     env = dict(os.environ, PYTHONPATH="")
-    r = subprocess.run([sys.executable, str(script), REF, ROOT], capture_output=True, text=True, timeout=600, env=env,
-                       cwd=str(tmp_path))
+    r = subprocess.run([sys.executable, str(script), str(checkout), ROOT], capture_output=True, text=True, timeout=600,
+                       env=env, cwd=str(tmp_path))
     assert r.returncode == 0, r.stdout[-3000:] + "\n" + r.stderr[-6000:]
     assert "OVERLAY_OK" in r.stdout
